@@ -2,6 +2,7 @@
 256x832 ResNet-18 on 1/2/4/8 B200; warp-loss HBM GB/s).
 
     python bench.py --gpus N --steps K --warmup W [--config kitti_r18|kitti_r50|nyu_r18]     # our arm (torchrun launches N>1)
+                    [--dump-outputs DIR]                                                      # + the last timed step's outputs
     python bench.py --impl reference --gpus N --steps K --warmup W                           # the reference's own CPU path
 
 A "step" is one complete optimisation step (train.py:254-282): 1 + n_ref DispResNet and 2 n_ref PoseResNet
@@ -297,11 +298,13 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps):
-        """device time of `steps` calls (L2 flushed before each), max over ranks, in ms"""
+    def timed(fn, steps, before=None):
+        """device time of `steps` calls (`before` run, then L2 flushed, ahead of each, outside the events), max over ranks, in ms"""
         evs = []
         barrier()
         for _ in range(steps):
+            if before is not None:
+                before()
             flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
@@ -359,6 +362,7 @@ def run_ours(args):
     L.PROF.update(enabled=False, only=None, events=[])
     del trainer
     trainer = make_trainer(args.conv_mode)
+    initial = trainer.optimizer.snapshot()      # seeded initialisation, no step taken yet
     for _ in range(2):
         trainer.step(d_tgt, d_refs, d_K)
 
@@ -381,13 +385,28 @@ def run_ours(args):
             return False
         return True
     graphed = capture(trainer)
+    # Every timed step starts from the seeded initial parameters and optimizer state, restored ahead of the step, before the L2
+    # flush and outside the timed events: the loss reductions and BatchNorm statistics accumulate with atomics, and a chain of
+    # Adam steps would carry their last-bit differences into everything after them.  So each timed step is the same work on
+    # the same values, run after run, and --dump-outputs can compare two builds output for output.
+    reset_launches = [0]
+
+    def reset():
+        n0 = L.launch_count()
+        trainer.optimizer.restore(initial)
+        for n in trainer.optimizer.nets:
+            n.refresh_operand_weights()        # the operand mirrors the next step reads (Adam writes them during replays)
+        reset_launches[0] += L.launch_count() - n0
     launches0 = L.launch_count()
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms = timed(lambda: trainer.step(d_tgt, d_refs, d_K), args.steps)
+    last = []
+    ms = timed(lambda: last.append(trainer.step(d_tgt, d_refs, d_K)), args.steps, before=reset)
     clocks = sampler.stop() if rank == 0 else None
-    launches = trainer.launches_per_step * args.steps if graphed else (L.launch_count() - launches0)
+    launches = trainer.launches_per_step * args.steps if graphed else (L.launch_count() - launches0 - reset_launches[0])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, trainer, last[-1])
 
     # ---- end to end: pinned host inputs copied in, loss read back, every step ----------------------
     result = torch.empty(4, dtype=torch.float32).pin_memory()
@@ -502,6 +521,29 @@ def run_ours(args):
     finish(world)
 
 
+DUMP_SAMPLE = 1 << 21
+
+
+def dump_outputs(out_dir, trainer, losses):
+    """What the last timed step computed, as float32 .npy files: losses.npy = (total, photo, smooth, geometry), the values
+    Trainer.step returns, and per network the parameter gradients of the step (disp_grads.npy, pose_grads.npy), flattened in
+    named_parameters order and shapes (the layout train.py checkpoints), each a fixed seeded sample of DUMP_SAMPLE elements
+    when larger (16 MiB in all).  The step starts from the seeded initial state (see the timed region), so two runs with the
+    same arguments agree to rounding.  The parameters after the Adam update are not written: an element whose gradient is
+    rounding noise moves by +-lr either way."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, t):
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    save("losses", torch.stack(losses))
+    for name, net in (("disp", trainer.disp_net), ("pose", trainer.pose_net)):
+        save(name + "_grads", torch.cat([p.grad.reshape(-1) for p in net.parameters() if p.grad is not None]))
+
+
 def finish(world):
     """End of a multi-rank run.  The captured CUDA graphs hold NCCL kernels: tearing the process group down with them alive
     hangs in the NCCL watchdog (observed on 2 GPUs: the line was printed, then destroy_process_group blocked until the
@@ -556,6 +598,8 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="time the eager step instead of the CUDA-graph replay")
     ap.add_argument("--overlap-wgrad", type=int, default=1, help="1 (default): weight gradients on a side stream per network (Trainer(overlap_wgrad=True))")
     ap.add_argument("--overlap-nets", type=int, default=1, help="1 (default): PoseResNet on a side stream next to DispResNet (Trainer(overlap_nets=True))")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the losses and parameter gradients of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -28,7 +28,11 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def golden_warp():
-    return np.load(os.path.join(GOLDEN, "warp_loss.npz"))
+    """warp_loss_{in,zeros,border,misc}.npz (make_golden.py stores the vectors in parts of under 1 MB) as one mapping."""
+    out = {}
+    for part in ("in", "zeros", "border", "misc"):
+        out.update(np.load(os.path.join(GOLDEN, "warp_loss_%s.npz" % part)))
+    return out
 
 
 @pytest.fixture(scope="session")

@@ -8,7 +8,7 @@ def t(a, dtype=torch.float32, device="cpu"):
 
 
 def golden_loss_inputs(g, dtype=torch.float32, device="cpu", n_scales=2, requires_grad=False):
-    """Rebuild the (tgt_img, ref_imgs, K, tgt_depth, ref_depths, poses, poses_inv) tuple of warp_loss.npz."""
+    """Rebuild the (tgt_img, ref_imgs, K, tgt_depth, ref_depths, poses, poses_inv) tuple of the golden warp / loss vectors."""
     def leaf(a):
         x = t(a, dtype, device)
         return x.requires_grad_(True) if requires_grad else x
@@ -59,15 +59,12 @@ def make_disk_dataset(root, H=128, W=160, scenes=("scene_a", "scene_b", "scene_v
 
 
 def reference_loader_env():
-    """Environment for a subprocess in which the reference's host-side loaders (datasets/*.py, custom_transforms.py: the
-    unmodified copy under baseline/_ref, plus the stand-ins for path / imageio under baseline/stubs) are importable from
-    PYTHONPATH, as train.py expects for real datasets.  None if baseline/_ref is absent (python __graft_entry__.py makes it)."""
+    """Environment for a subprocess in which host-side loaders with the reference's interface (datasets/*.py,
+    custom_transforms.py: the test doubles under tests/reference_loaders) are importable from PYTHONPATH, as train.py expects
+    for real datasets."""
     import os
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    ref, stubs = os.path.join(root, "baseline", "_ref"), os.path.join(root, "baseline", "stubs")
-    if not os.path.exists(os.path.join(ref, "datasets", "sequence_folders.py")):
-        return None
+    loaders = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_loaders")
     env = dict(os.environ)
-    env["PYTHONPATH"] = os.pathsep.join([stubs, ref] + ([env["PYTHONPATH"]] if env.get("PYTHONPATH") else []))
+    env["PYTHONPATH"] = os.pathsep.join([loaders] + ([env["PYTHONPATH"]] if env.get("PYTHONPATH") else []))
     env["PYTHONDONTWRITEBYTECODE"] = "1"
     return env

@@ -19,7 +19,7 @@ def _free_port():
     return p
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_data_parallel_step_matches_the_oracle_on_two_gpus():
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
            "--master-port", str(_free_port()), os.path.join(ROOT, "tests", "ddp_check.py")]

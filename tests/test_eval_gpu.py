@@ -154,16 +154,15 @@ def test_train_entry_end_to_end_on_synthetic_data(tmp_path, gpu_augment):
 
 @pytest.mark.parametrize("gpu_augment", [0, 1])
 def test_train_entry_on_a_dataset_on_disk(tmp_path, gpu_augment):
-    """`python train.py DIR ...` on a tiny JPEG dataset in the reference's folder layout, with the reference's own dataset
-    classes (unmodified copy under baseline/_ref) on PYTHONPATH as train.py expects: --gpu-augment 0 = the reference's host
-    transform chain in the loader, 1 = uint8 frames + the device-side transforms; training epoch, validation, checkpoints."""
+    """`python train.py DIR ...` on a tiny JPEG dataset in the reference's folder layout, with dataset classes of the
+    reference's interface (the test doubles under tests/reference_loaders) on PYTHONPATH as train.py expects: --gpu-augment 0 =
+    the host transform chain in the loader, 1 = uint8 frames + the device-side transforms; training epoch, validation,
+    checkpoints."""
     import os
     import subprocess
     import sys
     from helpers import make_disk_dataset, reference_loader_env
     env = reference_loader_env()
-    if env is None:
-        pytest.skip("baseline/_ref (copy of the reference made by __graft_entry__.build()) is not present")
     data = make_disk_dataset(str(tmp_path / "data"))
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     cmd = [sys.executable, os.path.join(root, "sc-sfmlearner-release_b200", "train.py"), data, "--name", "disk", "--epochs", "1",

@@ -7,9 +7,6 @@ import sys
 import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "baseline", "_ref")
-
 
 def test_save_checkpoint_layout_and_roundtrip(tmp_path):
     import models
@@ -29,24 +26,37 @@ def test_save_checkpoint_layout_and_roundtrip(tmp_path):
         assert w.is_contiguous() and tuple(w.shape) == (64, 64, 3, 3)      # plain OIHW tensors, not arena views
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "models", "DispResNet.py")), reason="baseline/_ref (copy of the reference) not installed")
 @pytest.mark.parametrize("layers", [18, 50])
-def test_checkpoints_load_into_the_unmodified_reference_modules(tmp_path, layers):
-    """The files train.py writes must be usable by the reference's test / inference scripts (strict load_state_dict into the
-    reference's own models.DispResNet / PoseResNet), in a clean interpreter so that the two `models` packages do not mix."""
+def test_checkpoints_load_into_the_unmodified_reference_modules(tmp_path, layers, golden_nets):
+    """The files train.py writes must be usable by the reference's test / inference scripts, i.e. load strictly into the
+    reference's own models.DispResNet / PoseResNet.  tests/golden/nets.npz holds, from the unmodified reference modules
+    (make_golden.py), their state_dict keys and shapes and their outputs for deterministic weights (one training-mode forward,
+    then eval mode with the running statistics it left): the checkpoint must carry exactly those keys and shapes, and loaded
+    strictly into the CPU port of the reference networks (oracle/nets.py) reproduce those outputs."""
+    import numpy as np
     import models
     import train as T
+    from golden_util import det_image, det_weights
+    from oracle import nets as N
     disp, pose = models.DispResNet(layers, False), models.PoseResNet(18, False)
+    for net in (disp, pose):
+        net.load_state_dict(det_weights(net.state_dict()))
     T.save_checkpoint(str(tmp_path), {"epoch": 1, "state_dict": disp.state_dict()}, {"epoch": 1, "state_dict": pose.state_dict()}, False)
-    code = ("import sys, torch; sys.dont_write_bytecode = True; sys.path.insert(0, %r); import models\n"
-            "d = models.DispResNet(%d, False); d.load_state_dict(torch.load(%r)['state_dict'])\n"
-            "p = models.PoseResNet(18, False); p.load_state_dict(torch.load(%r)['state_dict'])\n"
-            "x = torch.zeros(1, 3, 64, 96); d.eval(); p.eval()\n"
-            "print('OK', tuple(d(x).shape), tuple(p(x, x).shape))\n"
-            % (REF, layers, os.path.join(tmp_path, "dispnet_checkpoint.pth.tar"), os.path.join(tmp_path, "exp_pose_checkpoint.pth.tar")))
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stderr[-2000:]
-    assert "OK (1, 1, 64, 96) (1, 6)" in out.stdout
+    img1, img2 = det_image("img1", 2, 64, 96), det_image("img2", 2, 64, 96)
+    for prefix, tag, ref in (("dispnet", "disp%d" % layers, N.DispResNet(layers)), ("exp_pose", "pose18", N.PoseResNet(18))):
+        sd = torch.load(os.path.join(tmp_path, prefix + "_checkpoint.pth.tar"))["state_dict"]
+        assert list(sd.keys()) == list(golden_nets[tag + "_keys"])
+        assert ["x".join(map(str, v.shape)) for v in sd.values()] == list(golden_nets[tag + "_shapes"])
+        ref.load_state_dict(sd)                                 # strict
+        run = (lambda: ref(img1)) if prefix == "dispnet" else (lambda: ref(img1, img2))
+        ref.train()
+        with torch.no_grad():
+            out = run()
+        out, key = (out[0], "_out_s0") if prefix == "dispnet" else (out, "_out")
+        np.testing.assert_allclose(out.numpy(), golden_nets[tag + key], rtol=2e-4, atol=2e-5)
+        ref.eval()
+        with torch.no_grad():
+            np.testing.assert_allclose(run().numpy(), golden_nets[tag + "_eval_out"], rtol=2e-4, atol=2e-5)
 
 
 def test_cli_defaults_and_pretrained_weights(tmp_path, monkeypatch):
@@ -73,19 +83,18 @@ def test_cli_defaults_and_pretrained_weights(tmp_path, monkeypatch):
 
 
 def test_real_dataset_loaders_host_side(tmp_path):
-    """train.make_loaders on a dataset on disk with the reference's own dataset classes on PYTHONPATH: --gpu-augment 0 builds the
-    reference's host chain (normalised float tensors come out of the loader), --gpu-augment 1 builds the datasets with
-    transform=None and hands uint8 frames [B, n_img, H, W, 3] + intrinsics to the device stage (host side checked here, in a clean
-    interpreter; the device stage in tests/test_augment_gpu.py and tests/test_eval_gpu.py)."""
+    """train.make_loaders on a dataset on disk with dataset classes of the reference's interface on PYTHONPATH (the test doubles
+    under tests/reference_loaders): --gpu-augment 0 builds the host transform chain (normalised float tensors come out of the
+    loader), --gpu-augment 1 builds the datasets with transform=None and hands uint8 frames [B, n_img, H, W, 3] + intrinsics to
+    the device stage (host side checked here, in a clean interpreter; the device stage in tests/test_augment_gpu.py and
+    tests/test_eval_gpu.py)."""
     from helpers import make_disk_dataset, reference_loader_env
     env = reference_loader_env()
-    if env is None:
-        pytest.skip("baseline/_ref (copy of the reference made by __graft_entry__.build()) is not present")
     data = make_disk_dataset(str(tmp_path / "data"))
     pkg = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "sc-sfmlearner-release_b200")
     code = ("import sys; sys.path.insert(0, %r)\n"
             "import numpy as np, torch, train as T\n"
-            "SF = T._reference_dataset_module('sequence_folders'); assert 'baseline' in SF.__file__, SF.__file__\n"
+            "SF = T._reference_dataset_module('sequence_folders'); assert 'reference_loaders' in SF.__file__, SF.__file__\n"
             "for g in (0, 1):\n"
             "    args = T.parser.parse_args([%r, '--name', 'x', '-b', '2', '-j', '0', '--gpu-augment', str(g)])\n"
             "    class NoGpu(T.GpuAugmentLoader):\n"
